@@ -2,6 +2,7 @@
 """bench.py -- depth-maps/s of the PatchmatchNet cascade with the B200-native PatchMatch hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo (one JSON line on rank 0)
+    python bench.py ... --dump-outputs DIR                          # also write the last timed step's outputs as .npy
     python bench.py --impl reference [--steps K] [--warmup W]      # the reference algorithm on the host CPU
 
 Workload (BASELINE.json configs[1]): 1 reference + 4 source views, 640x512, full 3-stage cascade with
@@ -612,7 +613,8 @@ class Workload:
 
 def time_resident(wl, steps, flush, stream, barrier):
     """K steps with inputs resident in HBM: rounds of up to `slots` concurrent graph replays, L2 flushed before every
-    round outside the event pair that times it.  Returns the summed device seconds."""
+    round outside the event pair that times it.  Returns the summed device seconds; `wl.last_step` is left holding the
+    (depth, confidence) of the last step."""
     eng = wl.eng
     S = eng.n_slots
     rounds = [min(S, steps - r) for r in range(0, steps, S)]
@@ -622,9 +624,34 @@ def time_resident(wl, steps, flush, stream, barrier):
     for i, n_now in enumerate(rounds):
         flush()
         starts[i].record(stream)
-        eng.run_round(n_now, starts[i], ends[i])
+        wl.last_step = eng.run_round(n_now, starts[i], ends[i])[-1]
     barrier()
     return sum(s.elapsed_time(e) for s, e in zip(starts, ends)) * 1e-3
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy in float32.  When together they exceed DUMP_BYTES, each is replaced by
+    the same fixed, seeded sample of its flattened elements (a share of the budget proportional to its size), so
+    that two runs with the same arguments stay comparable element for element.  Returns what was written."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values()) * 4
+    written = {}
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        entry = {"shape": list(a.shape), "dtype": "float32"}
+        if total > DUMP_BYTES:
+            keep = max(1, a.size * DUMP_BYTES // total)
+            idx = np.sort(np.random.default_rng(0).choice(a.size, size=keep, replace=False))
+            a = a.reshape(-1)[idx]
+            entry["sample"] = f"{keep} of {t.numel()} elements, flat indices np.random.default_rng(0).choice({t.numel()}, {keep}, replace=False), sorted"
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
+        written[name] = entry
+    return written
 
 
 def time_e2e(wl, steps, stream, barrier):
@@ -716,7 +743,12 @@ def main() -> None:
     ap.add_argument("--cpu-samples", type=int, default=4)
     ap.add_argument("--repeats", type=int, default=5, help="the K-step timed region is repeated this many times; the line reports the median")
     ap.add_argument("--no-sub", action="store_true", help="skip the fp32 / 1600x1184 / batch-8 sub-records (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the depth map and confidence of the last timed step as DIR/<name>.npy "
+                         "(float32; rank 0; a fixed seeded sample when they exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -747,6 +779,7 @@ def main() -> None:
         dist = dist_mod
 
     B, N, H, W = args.batch, args.views, args.height, args.width
+    torch.manual_seed(0)  # the random depth hypotheses stage 3 draws on the GPU: the same arguments, the same outputs
     net, weights = build_net()
     wl = Workload(net, B, N, H, W, dev, args.slots, rank, use_graph=not args.no_graph)
     eng = wl.eng
@@ -789,6 +822,7 @@ def main() -> None:
     sampler.mark_begin()
     dev_runs = [time_resident(wl, args.steps, flush, stream, barrier) for _ in range(max(1, args.repeats))]
     sampler.mark_end()
+    last_step = {"depth": wl.last_step[0].cpu(), "confidence": wl.last_step[1].cpu()}  # before later phases reuse the slots
     clocks = sampler.stop()
     dev_runs = reduce_max(dev_runs)  # per repeat: the slowest rank
     dev_seconds = statistics.median(dev_runs)
@@ -915,6 +949,9 @@ def main() -> None:
             "gpu_eager_reference": gpu_eager,
         }
         line.update(sub)
+        if args.dump_outputs:
+            line["dumped_outputs"] = {"dir": args.dump_outputs, "step": "last timed step of the last repeat",
+                                      "arrays": dump_outputs(args.dump_outputs, last_step)}
         print(json.dumps(line), flush=True)
     if dist is not None:
         dist.destroy_process_group()

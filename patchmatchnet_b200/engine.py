@@ -14,7 +14,7 @@ There is no CPU path: construction fails without CUDA.
 """
 from __future__ import annotations
 
-from typing import Dict, Sequence, Tuple
+from typing import Dict, List, Sequence, Tuple
 
 import torch
 
@@ -138,17 +138,20 @@ class DepthEngine:
         with torch.no_grad():
             return self._forward(slot)
 
-    def run_round(self, n: int, start: torch.cuda.Event, done: torch.cuda.Event) -> None:
+    def run_round(self, n: int, start: torch.cuda.Event, done: torch.cuda.Event) -> List[Tuple[Tensor, Tensor]]:
         """`n` (<= n_slots) forwards concurrently, one per slot stream, fenced by `start` (already recorded on the
-        current stream) and `done` (recorded on the current stream once every slot has finished)."""
+        current stream) and `done` (recorded on the current stream once every slot has finished).  Returns each
+        forward's (depth, confidence), valid once `done` has completed."""
         cur = torch.cuda.current_stream(self.device)
+        outs = []
         for i in range(n):
             st = self._slots[i]["stream"]
             st.wait_event(start)
             with torch.cuda.stream(st):
-                self.run_slot(i)
+                outs.append(self.run_slot(i))
             cur.wait_stream(st)
         done.record(cur)
+        return outs
 
     # ------------------------------------------------------------------
     def upload(self, slot_idx: int, host: Dict[str, object], stream: torch.cuda.Stream) -> int:

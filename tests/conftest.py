@@ -11,7 +11,6 @@ REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if REPO not in sys.path:
     sys.path.insert(0, REPO)
 GOLDEN = os.path.join(REPO, "tests", "golden")
-REFERENCE = "/root/reference"
 
 warnings.filterwarnings("ignore", message="torch.meshgrid")
 warnings.filterwarnings("ignore", message=".*torch.jit.*is deprecated.*")
@@ -51,15 +50,10 @@ def golden_config1():
 
 
 @pytest.fixture(scope="session")
-def reference_models():
-    """The unmodified reference, importable only in the build container."""
-    if not os.path.isdir(os.path.join(REFERENCE, "models")):
-        pytest.skip("/root/reference not present (GPU box): oracle is pinned by the golden fixtures instead")
-    sys.path.insert(0, REFERENCE)
-    import models.net as ref_net
-    import models.patchmatch as ref_pm
-    import models.module as ref_mod
-    return ref_net, ref_pm, ref_mod
+def reference_net_calls():
+    """How the unmodified reference network (models/net.py) constructs and calls its three PatchMatch modules on
+    pm_cases.NET_CASE, every call's inputs and outputs, and its PatchMatch.forward schema (tests/golden/make_reference_golden.py)."""
+    return torch.load(os.path.join(GOLDEN, "net_calls.pt"), map_location="cpu")
 
 
 @pytest.fixture(scope="session")

@@ -86,6 +86,18 @@ def make_net_inputs(spec: Dict) -> Dict:
     return inp
 
 
+def warp_inputs():
+    """Inputs of the homography-warp / sampling-grid comparison: stage2_small's features and cameras, three depth
+    hypotheses per pixel (plane 0 behind the camera), and random offsets for the 16 propagation / 9 evaluation neighbours."""
+    case = make_stage_inputs(STAGE_CASES["stage2_small"])
+    B, _, H, W = case["ref_feature"].shape
+    g = torch.Generator().manual_seed(7)
+    depth = 400.0 + 600.0 * torch.rand(B, 3, H, W, generator=g)
+    depth[:, 0] = -50.0
+    offsets = {count: torch.randn(B, 2 * count, H * W, generator=g) for count in (16, 9)}
+    return case, depth, offsets
+
+
 def checksum(case: Dict) -> str:
     h = hashlib.sha256()
 

@@ -1,8 +1,7 @@
 """The drop-in boundary (SURVEY.md 8b): constructor / forward signatures, parameter names and shapes,
-error conventions -- checked without a GPU -- and, when the reference is importable, that our
-PatchMatch drops into the reference's UNMODIFIED models/net.py and loads its checkpoint."""
+error conventions -- checked without a GPU -- and that our PatchMatch takes the constructor and forward calls the
+reference's UNMODIFIED models/net.py makes and loads its checkpoint."""
 import inspect
-import sys
 
 import pytest
 import torch
@@ -72,19 +71,29 @@ def test_error_conventions_cpu():
             PatchMatch(evaluate_neighbors=10)(**kw)
 
 
-def test_drops_into_unmodified_reference_net(reference_models, golden_weights, monkeypatch):
-    """models/net.py binds PatchMatch by name at import (net.py:6); rebinding that one name swaps the hot path."""
-    ref_net, _, _ = reference_models
-    monkeypatch.setattr(ref_net, "PatchMatch", PatchMatch)
-    net = ref_net.PatchmatchNet(**pm_cases.NET_KWARGS)
-    assert all(type(getattr(net, f"patchmatch_{i}")) is PatchMatch for i in (1, 2, 3))
-    missing, unexpected = net.load_state_dict(golden_weights, strict=True)
-    assert not missing and not unexpected
-    net.eval()
-    inp = pm_cases.make_net_inputs(pm_cases.NET_CASE)
+def _recorded_kwargs(call):
+    return {k: (type(v)(t.clone() for t in v) if isinstance(v, (list, tuple)) else v.clone()) for k, v in call["inputs"].items()}
+
+
+def test_drops_into_unmodified_reference_net(reference_net_calls, golden_weights):
+    """models/net.py binds PatchMatch by name at import (net.py:6), so rebinding that one name swaps the hot path: the
+    class must accept the constructor keywords the reference network passes for each stage, load that stage's checkpoint
+    entries, and take the keyword call the network makes (all recorded from the unmodified reference)."""
+    rec = reference_net_calls
+    assert rec["forward_parameters"] == list(inspect.signature(PatchMatch.forward).parameters)[1:]
+    assert rec["state_keys"] == sorted(golden_weights)
+    mods = {}
+    for stage, kw in rec["ctor_kwargs"].items():
+        mods[stage] = PatchMatch(**kw)
+        missing, unexpected = mods[stage].load_state_dict(pm_cases.stage_state(golden_weights, stage), strict=True)
+        assert not missing and not unexpected
+        assert set(mods[stage].state_dict()) == {k[len(f"patchmatch_{stage}."):] for k in rec["state_keys"] if k.startswith(f"patchmatch_{stage}.")}
+    assert sorted(mods) == [1, 2, 3]
+    first = rec["calls"][0]
+    assert first["stage"] == 3
     with torch.no_grad(), pytest.raises(RuntimeError, match="no CPU fallback"):
-        # FeatureNet (reference code) runs; the first PatchMatch call refuses the CPU tensors
-        net(inp["images"], inp["intrinsics"], inp["extrinsics"], inp["depth_min"], inp["depth_max"])
+        # the first PatchMatch call of the reference's forward, on the CPU tensors it passed
+        mods[3].eval()(**_recorded_kwargs(first))
 
 
 def test_zero_copy_view_detection_needs_one_storage():

@@ -1,14 +1,14 @@
 """Geometric-consistency filtering (SURVEY.md 8f row f4; reference eval.py:86-190, :220-256).
 
 CPU: the oracle (oracle/geo_oracle.py) is pinned bit for bit against (a) cv2.remap for its restatement of the bilinear
-sampler, (b) the reference's own source text executed in the build container, (c) the committed reference-generated fixture.
+sampler, (b) what the reference's own source text computed on a seeded scene (tests/golden/geo_source_case.npz), (c) the
+committed reference-generated fixture.
 GPU (-m gpu): the one-launch kernel, through the C ABI, against the oracle and the fixture.  The masks are thresholded
 quantities: a pixel whose distance / relative depth difference lies within rounding of its threshold may legitimately flip
 (the kernel's float64 dot products are fused multiply-adds, BLAS's are not), so the bound is a fraction of pixels:
 <= 1e-4 of the pixels per mask, and the averaged depth must agree to 1e-6 relative wherever the masks agree."""
 import ctypes
 import os
-from typing import Tuple
 
 import numpy as np
 import pytest
@@ -18,11 +18,18 @@ from oracle import geo_oracle as go
 from tests import geo_cases
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "geo_case.npz")
+SOURCE_CASE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "geo_source_case.npz")
 
 
 @pytest.fixture(scope="module")
 def golden():
     z = np.load(GOLDEN)
+    return {k: z[k] for k in z.files}
+
+
+@pytest.fixture(scope="module")
+def source_case():
+    z = np.load(SOURCE_CASE)
     return {k: z[k] for k in z.files}
 
 
@@ -41,22 +48,18 @@ def test_remap_restatement_is_bit_exact_against_cv2():
     assert np.array_equal(want, go.remap_linear(img, mx, my))
 
 
-def test_oracle_is_bit_identical_to_the_reference_source():
-    cv2 = pytest.importorskip("cv2")
-    path = "/root/reference/eval.py"
-    if not os.path.exists(path):
-        pytest.skip("/root/reference not present (GPU box): the oracle is pinned by the golden fixture instead")
-    src = open(path).read()
-    ns = {"np": np, "cv2": cv2, "Tuple": Tuple}
-    exec(src[src.index("def reproject_with_depth("):src.index("def filter_depth(")], ns)  # eval.py:86-190, unmodified
+def test_oracle_is_bit_identical_to_the_reference_source(source_case):
+    """eval.py:86-190, executed unmodified from the reference's source text (tests/golden/make_reference_golden.py)."""
     sc = geo_cases.make_scene(seed=3, H=72, W=100, n_src=3)
-    for d, k, e in zip(sc["src_depths"], sc["src_Ks"], sc["src_Es"]):
-        rm, rd = ns["check_geometric_consistency"](sc["ref_depth"], sc["ref_K"], sc["ref_E"], d, k, e, 1.0, 0.01)
+    assert np.array_equal(sc["ref_depth"], source_case["ref_depth"]), "seeded scene differs from the one the fixture was made with"
+    for v, (d, k, e) in enumerate(zip(sc["src_depths"], sc["src_Ks"], sc["src_Es"])):
+        rm, rd = source_case[f"view{v}.mask"], source_case[f"view{v}.depth"]
         om, od = go.check_geometric_consistency(sc["ref_depth"], sc["ref_K"], sc["ref_E"], d, k, e, 1.0, 0.01)
         assert np.array_equal(rm, om) and np.array_equal(rd, od)
         assert 0.05 < rm.mean() < 0.95, "the scene must exercise both outcomes"
-        r3 = ns["reproject_with_depth"](sc["ref_depth"], sc["ref_K"], sc["ref_E"], d, k, e)
         o3 = go.reproject_with_depth(sc["ref_depth"], sc["ref_K"], sc["ref_E"], d, k, e)
+        r3 = [source_case[f"view{v}.reproject{i}"] for i in range(len(o3))]
+        assert f"view{v}.reproject{len(o3)}" not in source_case
         assert all(np.array_equal(a, b) for a, b in zip(r3, o3))
 
 
@@ -221,19 +224,12 @@ def _fusion_case(H, W, n_src, seed):
     return sc, final, np.where(np.isfinite(avg), avg, 0.0), img
 
 
-def test_fusion_oracle_is_bit_identical_to_the_reference_source():
-    path = "/root/reference/eval.py"
-    if not os.path.exists(path):
-        pytest.skip("/root/reference not present (GPU box)")
-    src = open(path).read().split("\n")
-    snippet = "\n".join(line[8:] for line in src[272:281])  # eval.py:273-281, the body of filter_depth's loop, de-indented
-    assert snippet.lstrip().startswith("height, width = depth_est_averaged.shape[:2]") and "vertex_colors.append" in snippet
+def test_fusion_oracle_is_bit_identical_to_the_reference_source(source_case):
+    """eval.py:273-281, the body of filter_depth's loop, executed from the reference's source text on this case."""
     sc, final, avg, img = _fusion_case(72, 100, 3, 3)
-    ns = dict(np=np, depth_est_averaged=avg, final_mask=final, ref_img=img, ref_intrinsics=sc["ref_K"], ref_extrinsics=sc["ref_E"],
-              vertices=[], vertex_colors=[])
-    exec(snippet, ns)
+    assert np.array_equal(final, source_case["fusion.final_mask"])
     v, c = go.fuse_points(final, avg, img, sc["ref_K"], sc["ref_E"])
-    assert 100 < len(v) < final.size and np.array_equal(ns["vertices"][0], v) and np.array_equal(ns["vertex_colors"][0], c)
+    assert 100 < len(v) < final.size and np.array_equal(source_case["fusion.vertices"], v) and np.array_equal(source_case["fusion.colors"], c)
 
 
 def _check_body(body, want_v, want_c):

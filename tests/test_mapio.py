@@ -1,13 +1,14 @@
 """Depth-map files (SURVEY.md 8f row f5; reference datasets/data_io.py:128-322): PFM and COLMAP .bin.
 
 Integer / byte work: the bar is bit-exact -- identical bytes on disk, identical arrays in memory.
-  oracle (oracle/mapio_oracle.py)  vs the unmodified reference functions (build container) and the reference-written
-                                   fixture files tests/golden/maps/* (everywhere);
+  oracle (oracle/mapio_oracle.py)  vs what the unmodified reference functions wrote and read
+                                   (tests/golden/maps/reference_cases.npz) and the reference-written fixture files tests/golden/maps/*;
   native (libpmb200.so through patchmatchnet_b200.data_io, the mirror of the reference's API)  vs the oracle, the
                                    fixtures and the reference; error texts as the reference raises them;
   -m gpu: file -> pinned buffer -> device and back."""
+import builtins
 import os
-import sys
+import re
 
 import numpy as np
 import pytest
@@ -33,12 +34,17 @@ def expected():
 
 @pytest.fixture(scope="module")
 def ref_io():
-    if not os.path.isdir("/root/reference/datasets"):
-        pytest.skip("/root/reference not present (GPU box): pinned by tests/golden/maps instead")
-    sys.path.insert(0, "/root/reference")
-    from datasets import data_io
+    """What the unmodified reference's save_map / save_pfm wrote and read_map / read_pfm returned for `_cases()`,
+    `SCALES` and `BAD_PFM` (tests/golden/make_reference_golden.py)."""
+    z = np.load(os.path.join(MAPS, "reference_cases.npz"))
+    return {k: z[k] for k in z.files}
 
-    return data_io
+
+SCALES = (1, 2.5, 0, 0.0, 1e-3, 123456.789)
+BAD_PFM = ((b"P6\n4 4\n-1.0\n" + bytes(64), Exception, "Not a PFM file."),
+           (b"Pf\n4  4\n-1.0\n" + bytes(64), Exception, "Malformed PFM header."),
+           (b"Pf\n4 4\n-1.0\n" + bytes(60), ValueError, "cannot reshape array of size 15 into shape"),
+           (b"Pf\n4 4\nabc\n" + bytes(64), ValueError, "could not convert string to float"))
 
 
 def _cases():
@@ -70,16 +76,15 @@ def test_oracle_reads_the_foreign_big_endian_fixture(expected):
     assert scale == 2.5 and _same(got, expected["foreign_be.pfm"])
 
 
-def test_oracle_matches_the_unmodified_reference(ref_io, tmp_path):
+def test_oracle_matches_the_unmodified_reference(ref_io):
     for tag, arr in _cases():
+        assert np.array_equal(ref_io[f"{tag}.input"], arr), tag
         for ext, enc in (("pfm", mo.encode_pfm), ("bin", mo.encode_bin)):
-            p = str(tmp_path / f"{tag}.{ext}")
-            ref_io.save_map(p, arr)
-            blob = open(p, "rb").read()
+            blob = ref_io[f"{tag}.{ext}.bytes"].tobytes()
             assert enc(arr) == blob, (tag, ext)
-            want = ref_io.read_map(p)
+            want = ref_io[f"{tag}.{ext}.read"]
             got = mo.decode_pfm(blob)[0] if ext == "pfm" else mo.decode_bin(blob)
-            assert _same(np.ascontiguousarray(want), got), (tag, ext)
+            assert _same(want, got), (tag, ext)
 
 
 # ---------------------------------------------------------------- native library (host code: runs on the CPU box too)
@@ -123,16 +128,16 @@ def test_native_matches_the_unmodified_reference_both_directions(ref_io, tmp_pat
         for ext in ("pfm", "bin"):
             mine, theirs = str(tmp_path / f"mine_{tag}.{ext}"), str(tmp_path / f"theirs_{tag}.{ext}")
             dio.save_map(mine, arr)
-            ref_io.save_map(theirs, arr)
+            with open(theirs, "wb") as f:
+                f.write(ref_io[f"{tag}.{ext}.bytes"].tobytes())
             assert open(mine, "rb").read() == open(theirs, "rb").read(), (tag, ext)
-            assert _same(dio.read_map(theirs), np.ascontiguousarray(ref_io.read_map(mine))), (tag, ext)
+            # (the bytes are equal, so the reference reads `mine` as it read its own file)
+            assert _same(dio.read_map(theirs), ref_io[f"{tag}.{ext}.read"]), (tag, ext)
     p = str(tmp_path / "scaled.pfm")
-    for scale in (1, 2.5, 0, 0.0, 1e-3, 123456.789):
+    for i, scale in enumerate(SCALES):
         dio.save_pfm(p, arr, scale)
-        mine = open(p, "rb").read()
-        ref_io.save_pfm(p, arr, scale)
-        assert mine == open(p, "rb").read(), scale
-        assert dio.read_pfm(p)[1] == ref_io.read_pfm(p)[1]
+        assert open(p, "rb").read() == ref_io[f"scaled{i}.bytes"].tobytes(), scale
+        assert dio.read_pfm(p)[1] == float(ref_io[f"scaled{i}.scale"])
 
 
 def test_empty_maps_round_trip(tmp_path):
@@ -182,17 +187,15 @@ def test_error_behaviour_follows_the_reference(tmp_path):
 
 def test_reference_raises_the_same_errors(ref_io, tmp_path):
     bad = tmp_path / "bad.pfm"
-    for blob, exc, text in ((b"P6\n4 4\n-1.0\n" + bytes(64), Exception, "Not a PFM file."),
-                            (b"Pf\n4  4\n-1.0\n" + bytes(64), Exception, "Malformed PFM header."),
-                            (b"Pf\n4 4\n-1.0\n" + bytes(60), ValueError, "cannot reshape array of size 15 into shape"),
-                            (b"Pf\n4 4\nabc\n" + bytes(64), ValueError, "could not convert string to float")):
+    for i, (blob, exc, text) in enumerate(BAD_PFM):
+        kind, message = str(ref_io[f"error{i}.type"]), str(ref_io[f"error{i}.message"])
+        assert issubclass(getattr(builtins, kind), exc) and re.search(text, message), (kind, message)
         bad.write_bytes(blob)
-        for fn in (ref_io.read_pfm, dio.read_pfm):
-            with pytest.raises(exc, match=text):
-                fn(str(bad))
+        with pytest.raises(exc, match=text):
+            dio.read_pfm(str(bad))
 
 
-def test_c_abi_rejects_bad_arguments():
+def test_c_abi_rejects_bad_arguments(tmp_path):
     from patchmatchnet_b200 import _native
 
     lib = _native.lib()
@@ -200,7 +203,7 @@ def test_c_abi_rejects_bad_arguments():
     assert lib.pmb200_map_probe(None, 1, info) == -1
     assert lib.pmb200_map_probe(b"/nonexistent/x.pfm", 7, info) == -1
     assert lib.pmb200_map_probe(b"/nonexistent/x.pfm", 1, info) == -3 and b"No such file" in lib.pmb200_last_error()
-    assert lib.pmb200_map_write(b"/tmp/x.pfm", 1, None, 4, 4, 2, 1.0) == -1
+    assert lib.pmb200_map_write(str(tmp_path / "x.pfm").encode(), 1, None, 4, 4, 2, 1.0) == -1
     p = os.path.join(MAPS, "depth_hw.pfm").encode()
     small = np.zeros(8, np.float32)
     assert lib.pmb200_map_read(p, 1, small.ctypes.data, 8, info) == -1 and b"too small" in lib.pmb200_last_error()

@@ -1,5 +1,9 @@
-"""Pin the oracle against the UNMODIFIED reference (build container only; skipped on the GPU box,
-where tests/test_golden.py pins it against fixtures the reference generated)."""
+"""Pin the oracle bit for bit against what the UNMODIFIED reference computed on the same inputs: its stage and network
+outputs (tests/golden/stage_cases.pt, net_case.pt, written by tests/golden/make_golden.py) and its warp and
+sampling-grid helpers (tests/golden/warp_case.pt, written by tests/golden/make_reference_golden.py).  The reference
+draws its random hypotheses from the global CPU generator; the oracle is seeded the same way."""
+import os
+
 import pytest
 import torch
 
@@ -7,11 +11,7 @@ from oracle import pm_oracle
 from patchmatchnet_b200.net import PatchmatchNet, load_reference_state
 from tests import pm_cases
 
-
-def _ref_stage(ref_pm, weights, stage):
-    mod = ref_pm.PatchMatch(**pm_cases.stage_ctor_kwargs(stage))
-    mod.load_state_dict(pm_cases.stage_state(weights, stage), strict=True)
-    return mod.eval()
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
 def _oracle_stage(weights, stage):
@@ -22,57 +22,49 @@ def _oracle_stage(weights, stage):
 
 
 @pytest.mark.parametrize("name", list(pm_cases.STAGE_CASES))
-def test_stage_bit_identical(reference_models, golden_weights, name):
-    _, ref_pm, _ = reference_models
+def test_stage_bit_identical(golden_weights, golden_stage_cases, name):
     spec = pm_cases.STAGE_CASES[name]
     case = pm_cases.make_stage_inputs(spec)
+    a = golden_stage_cases[name]
+    assert pm_cases.checksum(case) == a["checksum"], "seeded inputs differ from the ones the fixture was made with"
     kw = {k: case[k] for k in ("ref_feature", "src_features", "ref_proj", "src_projs", "depth_min", "depth_max", "depth", "view_weights")}
+    mod = _oracle_stage(golden_weights, spec["stage"])
     with torch.no_grad():
-        torch.manual_seed(spec["seed"] + 1000)
-        a = _ref_stage(ref_pm, golden_weights, spec["stage"])(**kw)
-        torch.manual_seed(spec["seed"] + 1000)
-        b = _oracle_stage(golden_weights, spec["stage"])(**kw)
-    for x, y in zip(a[0], b[0]):
+        torch.manual_seed(spec["seed"] + 1000)  # what the fixture's reference run drew from
+        b = mod(**kw)
+    assert len(a["depths"]) == len(b[0])
+    for x, y in zip(a["depths"], b[0]):
         assert torch.equal(x, y)
-    assert torch.equal(a[1], b[1]) and torch.equal(a[2], b[2])
+    assert torch.equal(a["score"], b[1]) and torch.equal(a["view_weights"], b[2])
 
 
-def test_warp_and_helpers_bit_identical(reference_models):
-    _, ref_pm, ref_mod = reference_models
-    case = pm_cases.make_stage_inputs(pm_cases.STAGE_CASES["stage2_small"])
+def test_warp_and_helpers_bit_identical():
+    want = torch.load(os.path.join(GOLDEN, "warp_case.pt"), map_location="cpu")
+    case, depth, offsets = pm_cases.warp_inputs()
     B, C, H, W = case["ref_feature"].shape
-    depth = 400.0 + 600.0 * torch.rand(B, 5, H, W)
-    depth[:, 0] = -50.0  # behind the camera -> exactly zero
-    a = ref_mod.differentiable_warping(case["src_features"][0], case["src_projs"][0], case["ref_proj"], depth)
     b = pm_oracle.homography_warp(case["src_features"][0], case["src_projs"][0], case["ref_proj"], depth)
-    assert torch.equal(a, b)
-    assert float(b[:, :, 0].abs().max()) == 0.0
+    assert torch.equal(want["warped"], b)
+    assert float(b[:, :, 0].abs().max()) == 0.0  # behind the camera -> exactly zero
     # neighbour tables + grid
-    mod = ref_pm.PatchMatch(**pm_cases.stage_ctor_kwargs(3))
-    for kind, gid, count in (("propagation", 1, 16), ("evaluation", 2, 9)):
-        off = torch.randn(B, 2 * count, H * W)
-        g_ref = mod.get_grid(gid, B, H, W, off, off.device)
-        g_or = pm_oracle.sampling_grid(pm_oracle.neighbour_table(kind, count, mod.dilation), off, H, W)
-        assert torch.equal(g_ref, g_or)
+    for kind, count in (("propagation", 16), ("evaluation", 9)):
+        g_or = pm_oracle.sampling_grid(pm_oracle.neighbour_table(kind, count, want["dilation"]), offsets[count], H, W)
+        assert torch.equal(want["grids"][kind], g_or)
 
 
-def test_full_network_bit_identical(reference_models, golden_weights):
-    ref_net, _, _ = reference_models
-    ref = ref_net.PatchmatchNet(**pm_cases.NET_KWARGS)
-    ref.load_state_dict(golden_weights, strict=True)
-    ref.eval()
+def test_full_network_bit_identical(golden_weights, golden_net_case):
     mine = PatchmatchNet(**pm_cases.NET_KWARGS, patchmatch_cls=pm_oracle.PatchMatchOracle)
     load_reference_state(mine, golden_weights)
     mine.eval()
     mine.stack_views = False  # the reference runs FeatureNet view by view
     inp = pm_cases.make_net_inputs(pm_cases.NET_CASE)
+    assert pm_cases.checksum(inp) == golden_net_case["checksum"]
     seed = pm_cases.NET_CASE["seed"] + 1000
     with torch.no_grad():
         torch.manual_seed(seed)
-        a = ref([i.clone() for i in inp["images"]], inp["intrinsics"].clone(), inp["extrinsics"].clone(), inp["depth_min"], inp["depth_max"])
-        torch.manual_seed(seed)
         b = mine([i.clone() for i in inp["images"]], inp["intrinsics"].clone(), inp["extrinsics"].clone(), inp["depth_min"], inp["depth_max"])
-    assert torch.equal(a[0], b[0]) and torch.equal(a[1], b[1])
-    for s in a[2]:
-        for x, y in zip(a[2][s], b[2][s]):
+    assert torch.equal(golden_net_case["depth"], b[0]) and torch.equal(golden_net_case["confidence"], b[1])
+    assert sorted(golden_net_case["per_stage"]) == sorted(b[2])
+    for s, ds in golden_net_case["per_stage"].items():
+        assert len(ds) == len(b[2][s])
+        for x, y in zip(ds, b[2][s]):
             assert torch.equal(x, y)

@@ -88,23 +88,28 @@ def test_scripted_module_is_inference_only(golden_weights):
         sm(*kw)
 
 
-def test_unmodified_reference_net_scripts_with_the_rebind(reference_models, golden_weights, monkeypatch, tmp_path):
-    """Exactly what train.py:50-55 does, with models.net.PatchMatch rebound: eval(), torch.jit.script, save; then
-    eval.py:38's torch.jit.load."""
-    ref_net, _, _ = reference_models
-    monkeypatch.setattr(ref_net, "PatchMatch", PatchMatch)
-    net = ref_net.PatchmatchNet(**pm_cases.NET_KWARGS)
-    net.load_state_dict(golden_weights, strict=True)
-    net.eval()
-    sm = torch.jit.script(net)
-    path = str(tmp_path / "module_000007.pt")
-    sm.save(path)
-    back = torch.jit.load(path)
-    assert "pmb200::warp_corr_score_" in str(back.patchmatch_3._forward_script.graph)
-    assert set(back.state_dict()) == set(golden_weights)
-    inp = pm_cases.make_net_inputs(pm_cases.NET_CASE)
-    with torch.no_grad(), pytest.raises(Exception):  # FeatureNet runs; the first pmb200 op has no CPU backend
-        back(inp["images"], inp["intrinsics"], inp["extrinsics"], inp["depth_min"], inp["depth_max"])
+def test_unmodified_reference_net_scripts_with_the_rebind(reference_net_calls, golden_weights, tmp_path):
+    """What train.py:50-55 does with models.net.PatchMatch rebound -- eval(), torch.jit.script, save; then eval.py:38's
+    torch.jit.load -- for each PatchMatch the reference network builds.  The network's scripted calls type-check against
+    the scripted forward: its arguments and result must be those of the reference's own PatchMatch (schema recorded)."""
+    rec = reference_net_calls
+    want = rec["forward_schema"]
+    for stage, kw in rec["ctor_kwargs"].items():
+        mod = PatchMatch(**kw)
+        mod.load_state_dict(pm_cases.stage_state(golden_weights, stage), strict=True)
+        sm = torch.jit.script(mod.eval())
+        schema = sm.forward.schema
+        assert [(a.name, str(a.type)) for a in schema.arguments[1:]] == want["arguments"]
+        assert [str(r.type) for r in schema.returns] == want["returns"]
+        path = str(tmp_path / f"patchmatch_{stage}.pt")
+        sm.save(path)
+        back = torch.jit.load(path)
+        assert "pmb200::warp_corr_score_" in str(back._forward_script.graph)
+        assert {f"patchmatch_{stage}.{k}" for k in back.state_dict()} == {k for k in golden_weights if k.startswith(f"patchmatch_{stage}.")}
+        if stage == 3:
+            call = {k: (list(v) if isinstance(v, tuple) else v) for k, v in rec["calls"][0]["inputs"].items()}
+            with torch.no_grad(), pytest.raises(Exception):  # the first pmb200 op has no CPU backend
+                back(**call)
 
 
 # ----------------------------------------------------------------------------------------------------------------
